@@ -2,7 +2,7 @@
 """Headline benchmark: Sigma-tiny forward images/s on synthetic 480x640 RGB-X (BASELINE.json), plus the
 selective-scan kernel's achieved fraction of the HBM roofline and the reference's CPU path timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl sigma|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl sigma|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one forward of the whole network over one batch of B images per GPU (weak scaling: every
@@ -12,7 +12,8 @@ rank runs its own B images, no data-path collective — the scan is per-sample, 
           and the logits of every step read back to the host, all inside the timed region; copies of neighbouring
           steps overlap the forward
   roofline / cpu_baseline : see DESIGN.md §Measurement.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  --dump-outputs DIR also writes, on rank 0, the logits of the last timed step of each arm
+(DIR/logits.npy for `value`, DIR/e2e_logits.npy for `e2e`, float32) so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -25,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
+sys.dont_write_bytecode = True     # the benchmark may run from a read-only tree: it writes nothing into it
 
 import torch  # noqa: E402
 
@@ -44,7 +46,7 @@ def parse():
                          "(BASELINE configs 3 / 4); default batch 2 per GPU")
     ap.add_argument("--amp", default="none", choices=["none", "bf16"], help="train mode: autocast dtype of the dense layers")
     ap.add_argument("--scan-impl", default="sigma", choices=["sigma", "ref_ext"],
-                    help="train mode: ref_ext swaps ONLY the native op for the reference's own CUDA extension (baseline/_ref) under the "
+                    help="train mode: ref_ext swaps ONLY the native op for the reference's own CUDA extension (oracle/_ref) under the "
                          "same composition = the reference's training step on this box (the GPU baseline of the training arm)")
     ap.add_argument("--composed", action="store_true",
                     help="train mode: CrossScan + einsum + op-level scan kernels (the round-1/2a training path) instead of the fused core")
@@ -64,7 +66,15 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-by-batch", action="store_true", help="skip the B = 1..16 sweep appended to the line at N = 1")
     ap.add_argument("--cpu-sample-images", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="infer mode: after the timed steps write the logits of the last timed step as DIR/logits.npy (resident "
+                         "inputs) and DIR/e2e_logits.npy (host inputs), float32 (B, classes, H, W); when the two would pass 64 MB, "
+                         "(B, classes, P) at P pixels drawn once with seed 0 (dump_pixels)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "sigma" or a.mode != "infer"):
+        ap.error("--dump-outputs writes the logits of the GPU forward: it needs --impl sigma --mode infer")
     if a.batch is None:
         a.batch = 74 if a.mode == "infer" else 2
     return a
@@ -206,6 +216,27 @@ class ClockSampler:
 
 
 
+# ------------------------------------------------------------------ --dump-outputs
+DUMP_BYTES = 64_000_000     # 64 MB for the dumped arrays together
+
+
+def dump_pixels(H, W, bytes_per_pixel):
+    """Flat pixel indices kept by --dump-outputs: None (all of them) when H·W pixels of `bytes_per_pixel` fit in DUMP_BYTES
+    (less room for the .npy headers), else a sorted sample drawn with seed 0, so every run at these arguments keeps the same."""
+    n = min(H * W, (DUMP_BYTES - 4096) // bytes_per_pixel)
+    if n == H * W:
+        return None
+    return torch.randperm(H * W, generator=torch.Generator().manual_seed(0))[:n].sort().values
+
+
+def dumped(logits, pix):
+    """(B, C, H, W) logits -> float32 host array, (B, C, P) at the pixels `pix` when it is not None."""
+    x = logits.detach().float()
+    if pix is not None:
+        x = x.reshape(x.shape[0], x.shape[1], -1)[:, :, pix.to(x.device)]
+    return x.cpu().numpy()
+
+
 # ------------------------------------------------------------------ GPU baseline: the reference's own CUDA extension
 REF_CALLS = {  # per image (SURVEY.md §8a1, App. B): name, KD, L, N, K, calls for tiny / small (base uses its own dims below)
     "enc0": (768, 19200, 16, 4, (4, 4)), "enc1": (1536, 4800, 16, 4, (4, 4)), "enc2": (3072, 1200, 16, 4, (18, 54)),
@@ -217,10 +248,10 @@ REF_CALLS = {  # per image (SURVEY.md §8a1, App. B): name, KD, L, N, K, calls f
 
 
 def measure_gpu_baseline(a, dev, batch=8):
-    """The reference's selective_scan_cuda_core rebuilt for sm_100a (baseline/_ref, recipe baseline/build_ref_ext.py) on the
+    """The reference's selective_scan_cuda_core rebuilt for sm_100a (oracle/_ref, recipe oracle/build_ref_ext.py) on the
     scan calls of one forward at 480x640 (synthetic tensors of the calls' shapes, `batch` images, best of nrows 1 / 4 as
     vmamba.py:183-191 would pick): aggregate algorithmic GB/s and ms per image — the GPU baseline the fused scan replaces."""
-    so = os.path.join(ROOT, "baseline", "_ref", "selective_scan_cuda_core.so")
+    so = os.path.join(ROOT, "oracle", "_ref", "selective_scan_cuda_core.so")
     if not os.path.exists(so) or a.model not in ("sigma_tiny", "sigma_small") or (a.height, a.width) != (480, 640):
         return None
     try:
@@ -383,7 +414,7 @@ def run_train(a):
         model = M.EncoderDecoder(cfg_of(a), criterion=torch.nn.CrossEntropyLoss(reduction="mean", ignore_index=255)).to(dev).train()
     if a.scan_impl == "ref_ext":
         ops.FUSED_TRAINING = False          # the GPU baseline is the reference's COMPOSITION over the reference's extension
-        sys.path.insert(0, os.path.join(ROOT, "baseline", "_ref"))
+        sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))
         import selective_scan_cuda_core as ref_ext
         ops.selective_scan_cuda_core_fwd = lambda u, delta, A, Bm, Cm, D=None, bias=None, sp=False, nrows=1, **k: ref_ext.fwd(u, delta, A, Bm, Cm, D, bias, sp, nrows)
         ops.selective_scan_cuda_core_bwd = lambda u, delta, A, Bm, Cm, D, bias, dout, x, sp, nrows=1, **k: ref_ext.bwd(u, delta, A, Bm, Cm, D, bias, dout if dout.stride(-1) == 1 else dout.contiguous(), x, sp, nrows)  # vmamba.py:72-74
@@ -667,10 +698,15 @@ def main():
     barrier()
     total_ms = sum(e0.elapsed_time(e1) for e0, e1 in ev)
     total_ms = dist_util.max_over_ranks(total_ms, dev)
+    dump = {}
+    if a.dump_outputs and rank == 0:     # before the e2e arm reuses the graph's static buffers
+        pix = dump_pixels(a.height, a.width, 2 * B * static_out.shape[1] * 4)
+        dump["logits"] = dumped(static_out, pix)
 
     # ---- timed region 2: end to end through the public call, host buffers
-    h_rgb = torch.randn(B, 3, a.height, a.width).pin_memory()
-    h_mx = torch.randn(B, 3, a.height, a.width).pin_memory()
+    gh = torch.Generator().manual_seed(dist_util.shard_seed(4321, rank))
+    h_rgb = torch.randn(B, 3, a.height, a.width, generator=gh).pin_memory()
+    h_mx = torch.randn(B, 3, a.height, a.width, generator=gh).pin_memory()
     h_outs = [torch.empty(tuple(static_out.shape), dtype=static_out.dtype).pin_memory() for _ in range(2)]
     cur = torch.cuda.current_stream()
     s0, s1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -708,6 +744,8 @@ def main():
         e2e_mode = "serial: H2D, forward, D2H on one stream"
     barrier()
     e2e_ms = dist_util.max_over_ranks(s0.elapsed_time(s1), dev)
+    if dump:
+        dump["e2e_logits"] = dumped(h_outs[(a.steps - 1) & 1] if pipe is not None else h_outs[0], pix)
     clocks = sampler.stop() if sampler else None
 
     if rank != 0:
@@ -811,6 +849,11 @@ def main():
         "gpu_launches": int(launches_per_step) * a.steps,
         "clocks": clocks,
     }
+    if dump:
+        import numpy as np
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,4 +1,4 @@
-"""Same box, same tensors: the reference CUDA extension rebuilt for sm_100a (baseline/_ref, recipe baseline/build_ref_ext.py)
+"""Same box, same tensors: the reference CUDA extension rebuilt for sm_100a (oracle/_ref, recipe oracle/build_ref_ext.py)
 next to sigma_b200's op-level kernels and the fused SS2D scan, on every a1 shape of SURVEY.md App. B.
 
     python scripts/bench_vs_ref_ext.py [--batch 1 8] [--dtypes f32 bf16] [--bwd] [--out gpurun_out/ref_ext_compare.json]
@@ -17,7 +17,7 @@ import sys
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path[:0] = [ROOT, os.path.join(ROOT, "baseline", "_ref")]
+sys.path[:0] = [ROOT, os.path.join(ROOT, "oracle", "_ref")]
 from sigma_b200 import _lib, fused, ops  # noqa: E402
 
 # name, KD, L, N, K, (fused kind, H, W, D, R) or None

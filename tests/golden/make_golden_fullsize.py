@@ -5,10 +5,11 @@
     python tests/golden/make_golden_fullsize.py base     # Sigma-base 720x960 B=1, 5 classes (config 5; odd 45->46->23 stage)
 
 Same recipe as make_golden.py (reference classes through ref_shim, procedural weights / inputs); because a
-full logits tensor is 11-14 MB, the fixture keeps: logits sub-sampled on a fixed 8x8 pixel lattice (all classes),
-the FULL arg-max map (uint8), the per-pixel top-2 logit margin quantised to fp16 (so a test can tell a flipped
-label at a near-tie from a real error), the 4 encoder stage outputs sub-sampled, and hist/mIoU from the
-reference's own utils/metric.py.
+full logits tensor is 11-14 MB and a fixture stays below 1 MB, it keeps: logits sub-sampled on a fixed pixel lattice
+(all classes; every 8th pixel, every 16th for the 40 classes of small; `logits_step`), the FULL arg-max map (uint8),
+the top-2 logit margin quantised to fp16 at the pixels where it is at most TIE of the logit scale (`tie_mask` packed
+bits, `tie_margin`; so a test can tell a flipped label at a near-tie from a real error), the 4 encoder stage outputs
+sub-sampled (`feat_step`), and hist/mIoU from the reference's own utils/metric.py.
 """
 import os
 import sys
@@ -30,6 +31,8 @@ CASES = {
     "small": ("sigma_small_480x640", "sigma_small", 480, 640, 40),
     "base": ("sigma_base_720x960", "sigma_base", 720, 960, 5),
 }
+STEPS = {"tiny": (8, 3), "small": (16, 3), "base": (8, 6)}   # logits lattice step, encoder-map spatial step
+TIE = 0.025                                                   # 2.5 x the largest logits bar of the tests (1e-2)
 
 
 @torch.no_grad()
@@ -62,12 +65,16 @@ def main():
         gt = (P.rand(SEED, tag + "/gt", (1, H, W)) * ncls).long().clamp(max=ncls - 1).numpy()
         hist, labeled, correct = hist_info(ncls, pred.numpy(), gt)
         iou, mean_iou, _, _, _, _ = compute_score(hist, correct, labeled)
-        out = dict(logits_sub=logits[:, :, 3::8, 5::8].contiguous().numpy(), argmax=pred.numpy().astype(np.uint8),
-                   margin=margin.numpy(), logits_absmax=np.float32(logits.abs().max()),
+        ls, fs = STEPS[which]
+        tie = (margin.float() <= TIE * logits.abs().max()).reshape(-1).numpy()
+        out = dict(logits_sub=logits[:, :, 3::ls, 5::ls].contiguous().numpy(), logits_step=np.asarray([3, 5, ls]),
+                   argmax=pred.numpy().astype(np.uint8), tie_bound=np.float32(TIE), tie_mask=np.packbits(tie),
+                   tie_margin=margin.reshape(-1).numpy()[tie], logits_absmax=np.float32(logits.abs().max()),
                    miou=np.float64(mean_iou), iou=np.asarray(iou), hist=np.asarray(hist),
                    ncalls=len(ns.stub.calls), dec_shape=np.asarray(dec_shape), ref_seconds=np.float64(dt))
+        out["feat_step"] = np.asarray([4, fs])
         for i, f in enumerate(feats):
-            out[f"feat{i}_sub"] = f[:, ::4, ::3, ::3].contiguous().numpy()
+            out[f"feat{i}_sub"] = f[:, ::4, ::fs, ::fs].contiguous().numpy()
             out[f"feat{i}_absmax"] = np.float32(f.abs().max())
         np.savez_compressed(os.path.join(HERE, tag + ".npz"), **out)
         print(tag, "mIoU", mean_iou, "scan calls", len(ns.stub.calls), f"{dt:.0f} s",

@@ -42,11 +42,16 @@ def test_library_has_no_runtime_dependency_on_cuda_libs(lib_path):
 def test_ctypes_binding_matches_header(lib_path):
     from sigma_b200 import _lib
     L = _lib.lib()
+    n0 = L.sigma_launch_count()        # GPU tests earlier in this process may have launched kernels
     assert L.sigma_abi_version() == 1
     assert set(_lib.SIGNATURES) >= _declared()
     assert L.sigma_ss2d_padded_cp(16, 6) == 40 and L.sigma_ss2d_padded_cp(4, 24) == 32 and L.sigma_ss2d_padded_cp(4, 65) == -1
     assert L.sigma_scan_fwd_workspace_bytes(2, 768, 1024, 16, 4, 0) > 0
-    assert L.sigma_launch_count() == 0
+    assert L.sigma_launch_count() == n0
+    # a freshly loaded library has launched nothing
+    r = subprocess.run([sys.executable, "-c", "import sys; sys.path.insert(0, %r); from sigma_b200 import _lib; print(_lib.launch_count())" % ROOT],
+                       capture_output=True, text=True)
+    assert r.returncode == 0 and r.stdout.split() == ["0"], r.stdout + r.stderr
 
 
 def test_sm100a_tma_in_sass(lib_path):
